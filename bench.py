@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- aggregated edges/s of the PNA layer forward on B200 (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over the whole graph: CSR (resident, built once) -> [N, 12*F] aggregation
@@ -19,6 +19,8 @@ N = 1: BASELINE.json configs[1] (ogbn-arxiv-shaped, 169 343 nodes / 1 166 243 ed
 N > 1: bench_multi.py -- configs[3] at N = 4 (graph-batch shard), configs[4] at N = 8 (destination partition + halo exchange),
        configs[4] at N/8 scale otherwise.
 --impl reference: the same workload's reference op sequence on the host cores (rank 0 only), same config / steps / warm-up.
+--dump-outputs DIR (N = 1): DIR/aggregate.npy, float32 rows of the last timed step's [N, 12*F] output (dump_rows says which),
+               so that two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -263,6 +265,22 @@ def side_configs(dev, flush, steps, peak):
     return res
 
 
+DUMP_LIMIT_BYTES = 64_000_000          # everything --dump-outputs writes, .npy header included
+
+
+def dump_rows(rowptr, row_bytes):
+    """Rows of the step's output that --dump-outputs writes: the whole output when it fits DUMP_LIMIT_BYTES, otherwise the
+    64 rows of largest in-degree (split across warps) plus a seeded random sample of the others, sorted.  A function of
+    the graph only, so every build writes the same rows."""
+    n = rowptr.numel() - 1
+    k = min(n, (DUMP_LIMIT_BYTES - 128) // row_bytes)
+    deg = (rowptr[1:] - rowptr[:-1]).cpu()
+    heavy = torch.sort(deg, descending=True, stable=True).indices[:min(64, k)]
+    rest = torch.randperm(n, generator=torch.Generator().manual_seed(0))
+    rest = rest[~torch.isin(rest, heavy)][:k - heavy.numel()]
+    return torch.sort(torch.cat([heavy, rest])).values
+
+
 def _rows_with_hubs(csr, n_sample):
     g = torch.Generator().manual_seed(11)
     rows = torch.randperm(csr.n_nodes, generator=g)[: min(n_sample, csr.n_nodes)]
@@ -333,6 +351,8 @@ def run_ours(args):
             step()
         torch.cuda.synchronize()
         per_step = bc.timed_steps(step, args.steps, args.warmup, flush)
+        if args.dump_outputs:                       # before the untimed passes below overwrite `out`
+            dumped = out[dump_rows(csr.rowptr, out.size(1) * out.element_size()).to(dev)].cpu()
         t_end = time.perf_counter() + 0.5
         while time.perf_counter() < t_end:
             step()
@@ -464,6 +484,10 @@ def run_ours(args):
         "cpu_baseline": cpu,
         "configs": sides,
     }
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "aggregate.npy"), dumped.numpy())
     print(json.dumps(line))
 
 
@@ -475,7 +499,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU leg (profiling runs)")
     ap.add_argument("--no-side-configs", action="store_true", help="skip the `configs` sub-object (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rows of the last timed step's output to DIR/aggregate.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs: --impl ours on one GPU only")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)

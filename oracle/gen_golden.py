@@ -1,6 +1,6 @@
 """Generate tests/golden/*.pt by RUNNING THE REFERENCE'S OWN FILES in the authoring container.
 
-    PYTHONPATH=. python oracle/gen_golden.py            (needs /root/reference; not runnable on the GPU box)
+    PNA_REFERENCE=<reference checkout> PYTHONPATH=. python oracle/gen_golden.py [--round2 | --propagate]
 
 /root/reference's PyG and DGL layers import torch_geometric / torch_scatter / dgl, none of which exist here; they are
 imported over the minimal third-party restatements in oracle/shims/ (see its README).  The files under test --
@@ -242,10 +242,28 @@ def round2_cases():
                                   posttrans_layers=1, divide_input=True), state_dict=layd.state_dict(), out=outd))
 
 
+def propagate_case():
+    """PNAConvSimple.propagate alone on a random multigraph, example.py's aggregator order: the aggregation the oracle
+    restates, pinned bit for bit by tests/test_oracle.py."""
+    torch.manual_seed(5)
+    n, e, f = 300, 2000, 24
+    x = torch.randn(n, f)
+    ei = torch.randint(0, n, (2, e))
+    deg = deg_hist(ei[1], n)
+    conv = PNAConvSimple(f, f, A4_EX, S3, deg)
+    with torch.no_grad():
+        agg = conv.propagate(ei, x=x, size=None)
+    save("pyg_propagate_f24", dict(kind="pyg_propagate", x=x, edge_index=ei, deg=deg, aggregators=A4_EX, scalers=S3,
+                                   avg_deg=conv.avg_deg, aggregate=agg))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     if "--round2" in sys.argv:
         round2_cases()
+        sys.exit(0)
+    if "--propagate" in sys.argv:
+        propagate_case()
         sys.exit(0)
     simple_case("pyg_simple_f16", 200, 900, 16, seed=1)
     simple_case("pyg_simple_f64_hub", 100, 400, 64, seed=2, hub=700)

@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
 import threading
 
@@ -40,6 +41,12 @@ FLAG_ZERO_ISOLATED, FLAG_SKIP_LIGHT, FLAG_SKIP_HUBS, FLAG_RELU_VAR, FLAG_GATHER_
 EXPORTED_SYMBOLS = ("pna_csr_workspace_bytes", "pna_csr_build", "pna_csr_light_view", "pna_csr_light_view_workspace_bytes", "pna_aggregate_fwd", "pna_aggregate_bwd",
                     "pna_aggregate_bwd_coef", "pna_aggregate_bwd_combine",
                     "pna_gather_rows", "pna_halo_pull", "pna_peer_barrier", "pna_linear_fwd", "pna_linear_scaled_fwd", "pna_row_scales", "pna_linear_workspace_bytes", "pna_query", "pna_last_error")
+
+
+def cuda_tool(name: str) -> str:
+    """Path of a CUDA toolkit program (nvcc, cuobjdump): PATH first, then $CUDA_HOME/bin (default /usr/local/cuda), so that
+    the build does not depend on the caller's shell having the toolkit on PATH."""
+    return shutil.which(name) or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", name)
 
 
 class PnaError(RuntimeError):
@@ -105,7 +112,7 @@ def build_library(force: bool = False, verbose: bool = False, extra_flags=()) ->
         objs.append(obj)
         stale = force or not os.path.exists(obj) or os.path.getmtime(obj) < max(os.path.getmtime(src), hdr_time)
         if stale:
-            jobs.append(["nvcc"] + NVCC_FLAGS + list(extra_flags) + ["-c", src, "-o", obj])
+            jobs.append([cuda_tool("nvcc")] + NVCC_FLAGS + list(extra_flags) + ["-c", src, "-o", obj])
 
     def run(cmd):
         if verbose:
@@ -118,7 +125,7 @@ def build_library(force: bool = False, verbose: bool = False, extra_flags=()) ->
     with ThreadPoolExecutor(max_workers=min(8, os.cpu_count() or 1)) as ex:
         logs = list(ex.map(run, jobs))
     if jobs or not os.path.exists(LIB_PATH) or os.path.getmtime(LIB_PATH) < max(os.path.getmtime(o) for o in objs):
-        run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", LIB_PATH] + objs)
+        run([cuda_tool("nvcc"), "-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-o", LIB_PATH] + objs)
     if verbose and extra_flags:
         print("\n".join(logs))
     return LIB_PATH

@@ -42,7 +42,7 @@ def test_struct_layouts_match_the_header():
 
 def test_library_targets_sm_100a_only():
     import subprocess
-    out = subprocess.run(["cuobjdump", "--list-elf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    out = subprocess.run([_lib.cuda_tool("cuobjdump"), "--list-elf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

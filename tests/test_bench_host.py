@@ -99,3 +99,19 @@ def test_parity_checker_accepts_the_oracle_and_rejects_a_corrupted_row():
     assert not bc.sampled_parity(bad, rowptr, col, lambda idx: x[idx], big_row_edges=1000, big_row_cols=4, **kw)["ok"]
     # wrong source features (what a broken halo exchange would look like) are caught too
     assert not bc.sampled_parity(out, rowptr, col, lambda idx: x[(idx + 1) % n], **kw)["ok"]
+
+
+def test_dump_rows_are_fixed_include_the_heaviest_and_fit_the_limit():
+    """bench.py --dump-outputs: every row when the output fits, else a fixed sample holding the 64 largest in-degrees."""
+    import bench
+    src, dst = _graph()
+    n = 300
+    deg = torch.bincount(dst, minlength=n)
+    rowptr = torch.cat([torch.zeros(1, dtype=torch.long), torch.cumsum(deg, 0)])
+    assert torch.equal(bench.dump_rows(rowptr, 4 * 1536), torch.arange(n))
+    row_bytes = bench.DUMP_LIMIT_BYTES // 100
+    rows = bench.dump_rows(rowptr, row_bytes)
+    assert rows.numel() == 99 and rows.numel() * row_bytes + 128 <= bench.DUMP_LIMIT_BYTES
+    assert torch.equal(rows, torch.unique(rows)) and torch.equal(rows, bench.dump_rows(rowptr, row_bytes))
+    heavy = torch.sort(deg, descending=True, stable=True).indices[:64]
+    assert bool(torch.isin(heavy, rows).all()) and 11 in rows.tolist()

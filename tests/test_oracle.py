@@ -1,6 +1,5 @@
 """Pin oracle/pna_oracle.py against outputs of the reference's own files (tests/golden, made by oracle/gen_golden.py)."""
 import math
-import os
 
 import pytest
 import torch
@@ -28,8 +27,13 @@ def test_simple_layer_forward(name):
     lay = O.PNAConvSimpleOracle(f, f, g["aggregators"], g["scalers"], g["deg"], post_layers=g["post_layers"])
     lay.load_state_dict(g["state_dict"])
     with torch.no_grad():
+        agg = lay.propagate(g["x"], g["edge_index"])
         out = lay(g["x"], g["edge_index"])
-    assert torch.equal(out, g["out"])
+    assert torch.equal(agg, g["aggregate"])
+    # The post-MLP is a CPU GEMM (K = 12 F, up to 900) whose fp32 summation order depends on the instruction set and the
+    # thread count: the stored output is reproduced bit for bit only by the configuration that stored it (measured: up to
+    # 1e-6 apart between thread counts of one CPU).  Bar: the 1e-5 fp32 layer bar the GPU path meets on these fixtures.
+    torch.testing.assert_close(out, g["out"], rtol=1e-5, atol=1e-5)
 
 
 @pytest.mark.parametrize("name", CONV)
@@ -120,23 +124,14 @@ def test_k3_analytic_rows():
     torch.testing.assert_close(out[1], torch.cat([base, base * amp, base * att]), rtol=1e-6, atol=1e-7)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference checkout not on this machine")
-def test_live_reference_over_shims():
-    """In the authoring container, re-run the real reference file and compare with the oracle on fresh inputs."""
-    import subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = (
-        "import torch\n"
-        "from models.pytorch_geometric.pna import PNAConvSimple\n"
-        "from oracle import pna_oracle as O\n"
-        "torch.manual_seed(5); n,e,f=300,2000,24\n"
-        "x=torch.randn(n,f); ei=torch.randint(0,n,(2,e)); deg=torch.bincount(torch.bincount(ei[1],minlength=n))\n"
-        "A=['mean','min','max','std']; S=['identity','amplification','attenuation']\n"
-        "c=PNAConvSimple(f,f,A,S,deg); r=c.propagate(ei,x=x,size=None)\n"
-        "assert torch.equal(r,O.simple_propagate(x,ei,A,S,c.avg_deg)); print('ok')\n")
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(root, "oracle", "shims"), "/root/reference", root]))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=root)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stderr
+def test_reference_propagate_over_shims():
+    """The reference's PNAConvSimple.propagate, run over oracle/shims on random inputs (tests/golden/pyg_propagate_f24,
+    made by oracle/gen_golden.py --propagate), equals the oracle bit for bit, with the reference's own avg_deg."""
+    g = load_golden("pyg_propagate_f24")
+    agg = O.simple_propagate(g["x"], g["edge_index"], g["aggregators"], g["scalers"], g["avg_deg"])
+    assert torch.equal(agg, g["aggregate"])
+    mine = O.avg_deg_from_histogram(g["deg"])
+    assert mine["lin"] == g["avg_deg"]["lin"] and mine["log"] == g["avg_deg"]["log"]
 
 
 def test_c_oracle_agrees_with_torch_oracle():
